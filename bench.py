@@ -29,6 +29,10 @@ Inputs (20 GB) are far larger than L2 (126 MB), so every step streams from HBM; 
              g++ -O3 -march=native (AVX-512 where present), one pinned thread per hardware thread —
              plus `arrow_compute`: the same predicate through pyarrow.compute (not Gandiva either).
 `--impl reference` prints that CPU arm as its own line (same workload, same rows per step).
+
+`--dump-outputs DIR` writes the SelectionVector of the last timed step to DIR as float64 .npy files
+(see dump_outputs), so that two builds run with the same arguments can be compared output for output.
+The bench writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -91,7 +95,12 @@ def parse_args():
     ap.add_argument("--sm-reserve", type=int, default=-1,
                     help="SMs the filter leaves free for the push / NCCL kernels (default with N>1: 2, i.e. twelve "
                          "256-thread CTA slots for the eight push CTAs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the SelectionVector of the last timed step to DIR (float64 .npy, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peak_gbs():
@@ -688,7 +697,33 @@ def gpu_numa_cpus(torch, dev):
         return None, None
 
 
+DUMP_SAMPLE = 3 << 20    # entries kept of a longer SelectionVector: 2 x 24 MB with their positions
+
+
+def dump_outputs(directory, vec, count):
+    """--dump-outputs: the SelectionVector a caller of the timed path receives (`count` row numbers, ascending)
+    as float64, exact below 2**53.  selection_count.npy holds the count; selection_vector.npy the vector, or,
+    when it is longer than 2 x DUMP_SAMPLE entries, the entries at DUMP_SAMPLE positions drawn with a fixed
+    seed, which selection_positions.npy holds.  At most 48 MB in all."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    idx = vec[:count].to(torch.int64)
+    if vec.dtype == torch.int32:                  # UINT32 entries live in an int32 tensor
+        idx &= 0xFFFFFFFF
+    np.save(os.path.join(directory, "selection_count.npy"), np.array([count], dtype=np.float64))
+    positions = os.path.join(directory, "selection_positions.npy")
+    if idx.numel() > 2 * DUMP_SAMPLE:
+        pos = np.sort(np.random.default_rng(0).choice(idx.numel(), DUMP_SAMPLE, replace=False))
+        idx = idx[torch.from_numpy(pos).to(idx.device)]
+        np.save(positions, pos.astype(np.float64))
+    elif os.path.exists(positions):              # left by an earlier, sampled run
+        os.remove(positions)
+    np.save(os.path.join(directory, "selection_vector.npy"), idx.cpu().numpy().astype(np.float64))
+
+
 def main():
+    sys.dont_write_bytecode = True   # no __pycache__ in the tree, which may be read-only
     args = parse_args()
     if args.impl == "reference":
         run_reference(args)
@@ -729,6 +764,8 @@ def main():
     idx_mode = "UINT32" if (world == 1 and n <= (1 << 32)) else "UINT64"
     idx_dtype = torch.int32 if idx_mode == "UINT32" else torch.int64
     use_push = world > 1 and not args.no_gather and args.gather == "push"
+    if args.dump_outputs and world > 1 and not use_push:
+        raise SystemExit("--dump-outputs with N>1 needs --gather push (the vector a caller receives is rank 0's)")
     sm_reserve = args.sm_reserve if args.sm_reserve >= 0 else ((2 if use_push else 4) if world > 1 and not args.no_gather else 0)
     cfg = gandiva.Configuration(device=local_rank, rows_per_thread=args.rows_per_thread,
                                 block_threads=args.block_threads, sm_reserve=sm_reserve)
@@ -986,6 +1023,9 @@ def main():
             for j in range(waves):
                 dist.send(mine[j], dst=0)
         del mine
+    if args.dump_outputs and rank == 0:             # before the kernel-only timing below reuses out_idx
+        vec, total = ps.result(gstep["i"] - 1) if use_push else (out_idx, count)
+        dump_outputs(args.dump_outputs, vec, total)
 
     # ---- roofline of the dominant (only) kernel ----------------------------------------------
     peak, peak_src = measured_peak_gbs()

@@ -6,7 +6,9 @@ BENCH / TEST INFRASTRUCTURE ONLY (see oracle/__init__.py): imported by bench.py'
 The library is compiled on first use ON THE MACHINE THAT RUNS IT with `g++ -O3 -march=native`
 (`oracle/_proxy/libgdv_cpu_proxy_<cpu-flags-hash>.so`, git-ignored): a `.so` built in the GPU-less
 container travels to the GPU box, whose host CPU may have a different instruction set, so the file
-name carries a hash of /proc/cpuinfo's flags and a mismatch triggers a one-second rebuild.
+name carries a hash of /proc/cpuinfo's flags and a mismatch triggers a one-second rebuild.  The build step
+(gandiva_b200/build.py) writes the in-tree file; a rebuild at run time goes to the temporary directory
+(`gdv_cpu_proxy_<uid>/`), so that the benchmark also runs from a read-only tree.
 """
 from __future__ import annotations
 
@@ -14,6 +16,7 @@ import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -35,10 +38,10 @@ def _cpu_key() -> str:
     return hashlib.sha1(flags.encode() + src).hexdigest()[:12]
 
 
-def build() -> str:
-    path = os.path.join(_DIR, "libgdv_cpu_proxy_%s.so" % _cpu_key())
+def build(directory: str = _DIR) -> str:
+    path = os.path.join(directory, "libgdv_cpu_proxy_%s.so" % _cpu_key())
     if not os.path.exists(path):
-        os.makedirs(_DIR, exist_ok=True)
+        os.makedirs(directory, exist_ok=True)
         tmp = path + ".tmp%d" % os.getpid()
         subprocess.check_call(["g++"] + CXXFLAGS + [os.path.join(_HERE, "cpu_proxy.cc"), "-o", tmp])
         os.replace(tmp, path)
@@ -51,7 +54,10 @@ _lib = None
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        L = C.CDLL(build())
+        path = os.path.join(_DIR, "libgdv_cpu_proxy_%s.so" % _cpu_key())
+        if not os.path.exists(path):   # a CPU the in-tree build did not see: the tree may be read-only
+            path = build(os.path.join(tempfile.gettempdir(), "gdv_cpu_proxy_%d" % os.getuid()))
+        L = C.CDLL(path)
         vp, i64 = C.c_void_p, C.c_int64
         L.proxy_threads.restype = C.c_int
         L.proxy_threads.argtypes = [C.c_int]
